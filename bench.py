@@ -441,7 +441,13 @@ def run_gpu_arm(args):
     torch.cuda.synchronize()
     ops.check_index_errors()
     l0 = lib.raw("dv3_launch_count")()
-    t_res = timed(lambda: step.step(resident), args.steps)
+    last = {}
+
+    def timed_step():
+        last["loss"] = step.step(resident)
+    t_res = timed(timed_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["loss"], step.model)
     launches = (lib.raw("dv3_launch_count")() - l0) // args.steps
     if step.launches_per_step is not None:       # graph replay: the launches were recorded at capture time
         launches = step.launches_per_step
@@ -602,6 +608,21 @@ def run_gpu_arm(args):
         dist.destroy_process_group()
 
 
+DUMP_PARAMS = 8 << 20          # parameters sampled into params_sample.npy: 32 MB of float32
+
+
+def dump_outputs(out_dir, loss, model):
+    """What the last timed step hands its caller: the loss (loss.npy, float64) and the updated parameters -- the
+    parameters in model.parameters() order, flattened, at a fixed seeded sample of DUMP_PARAMS positions in
+    increasing order (params_sample.npy, float32)."""
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters()])
+    n = flat.numel()
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:min(n, DUMP_PARAMS)].sort().values
+    np.save(os.path.join(out_dir, "loss.npy"), np.float64(loss.double().item()))
+    np.save(os.path.join(out_dir, "params_sample.npy"), flat[idx.to(flat.device)].float().cpu().numpy())
+
+
 def stft_throughput(dev, world, rank, timed):
     """BASELINE.json config #5 (10k synthetic 10 s clips @22.05 kHz), sharded round-robin over the ranks with no
     collective: every rank processes ceil(10000 / world) clips as resident batches of 256 -> clips/s of the whole job,
@@ -650,6 +671,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the sub-benchmarks (other presets, STFT, exact-fp32 mode, reference-in-eager competitor)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and a fixed sample of the updated parameters of the "
+                         "last timed step to DIR/*.npy (same arguments -> same inputs, for comparing two builds)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)

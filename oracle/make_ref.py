@@ -11,10 +11,9 @@ the GPU box, where /root/reference does not exist.  Consumers (all test / bench 
 
 * ``bench.py --impl reference``      the reference's own modules + losses + Adam on the host CPU (kind "reference")
 * ``bench.py`` ``gpu_eager_baseline``  the same modules through PyTorch eager (cuDNN/cuBLAS) on the B200
-* ``tests/test_gpu_dropin.py``       reference ``train.py`` (``build_model`` / ``train`` / ``collate_fn``) executed
-                                     UNCHANGED on top of ``deepvoice3_pytorch_b200`` (``oracle/ref_harness.py``)
 * ``tests/golden/make_train_golden.py``  fixtures for the loss / collate functions of ``train.py``
-* ``tests/test_dropin.py``           also runs reference ``synthesis.py``'s ``tts()`` UNCHANGED on this package
+* ``tests/golden/make_dropin_golden.py``  fixtures of ``train.py`` / ``synthesis.py`` / ``ljspeech.py`` run on the
+                                          reference package, for ``tests/test_dropin.py``
 """
 import os
 import shutil

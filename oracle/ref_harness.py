@@ -1,4 +1,4 @@
-"""TEST / BENCH INFRASTRUCTURE -- loads the reference's own ``train.py`` (from ``oracle/_ref`` or /root/reference) UNCHANGED,
+"""TEST / BENCH INFRASTRUCTURE -- loads the reference's own ``train.py`` (from ``oracle/_ref``) UNCHANGED,
 on top of either the reference package or ``deepvoice3_pytorch_b200``.
 
 ``train.py`` imports a number of packages that are not installed here and that the training hot path never touches
@@ -23,14 +23,9 @@ N_VOCAB = 149          # len(symbols) of the reference's English frontend (front
 
 
 def ref_root():
-    """oracle/_ref when built/shipped, else the read-only reference tree (build container)."""
-    p = os.path.join(HERE, "_ref")
-    if os.path.isdir(os.path.join(p, "deepvoice3_pytorch")):
-        return p
-    if os.path.isdir("/root/reference/deepvoice3_pytorch"):
-        from oracle import make_ref
-        return make_ref.build(quiet=True)
-    return None
+    """oracle/_ref when it has been built (oracle/make_ref.py), else None."""
+    from oracle import make_ref
+    return make_ref.path()
 
 
 class _Missing(types.ModuleType):

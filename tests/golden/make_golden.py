@@ -25,6 +25,8 @@ import torch
 warnings.filterwarnings("ignore")
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = "/root/reference"
+sys.path.insert(0, os.path.dirname(HERE))
+import golden_util as G  # noqa: E402
 
 
 def import_reference():
@@ -49,9 +51,7 @@ class Fixture:
         self.d["%s|%s|%s" % (case, group, name)] = t2n(value) if torch.is_tensor(value) else np.asarray(value)
 
     def save(self, fname):
-        path = os.path.join(HERE, fname)
-        np.savez_compressed(path, **self.d)
-        print("wrote %s: %d arrays, %.1f KB" % (fname, len(self.d), os.path.getsize(path) / 1024))
+        G.save(fname, self.d)
 
 
 def loss_weights(shape, i):
@@ -355,7 +355,6 @@ def init_fingerprints():
     """Same torch seed -> same initial weights: per-tensor (sum, abs-sum, first element) of the reference
     builders' freshly initialised models at the three BASELINE.json presets (seed 4321)."""
     from deepvoice3_pytorch import builder
-    sys.path.insert(0, os.path.dirname(HERE))
     from test_gpu_models import preset_kwargs
     fx = Fixture()
     for preset in ["deepvoice3_ljspeech", "nyanko_ljspeech", "deepvoice3_vctk"]:

@@ -4,7 +4,7 @@
 
     python tests/golden/make_train_golden.py          (build container: needs /root/reference)
 
-Writes tests/golden/train_fns.npz:
+Writes tests/golden/train_fns.*.npz:
 
 * ``mask*``      ``sequence_mask`` (train.py:261-271)
 * ``specloss*``  ``spec_loss`` (train.py:547-582) incl. the priority-bin branch (:559-567) and w = 0 / bw = 0 corners
@@ -26,7 +26,9 @@ warnings.filterwarnings("ignore")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 from oracle import ref_harness as H  # noqa: E402
+import golden_util as G  # noqa: E402
 
 OUT = {}
 
@@ -146,9 +148,7 @@ def main():
         for k, p in (("mel_out", model.mel), ("lin_out", model.lin), ("attn", model.attn), ("done_hat", model.done)):
             put(name, "out", "grad_" + k, p.grad if p.grad is not None else torch.zeros_like(p))
 
-    path = os.path.join(HERE, "train_fns.npz")
-    np.savez_compressed(path, **OUT)
-    print("wrote %s: %d arrays, %.1f KB" % (path, len(OUT), os.path.getsize(path) / 1024))
+    G.save("train_fns.npz", OUT)
 
 
 if __name__ == "__main__":

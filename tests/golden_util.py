@@ -1,4 +1,6 @@
-"""Loader for the golden vectors written by tests/golden/make_golden.py."""
+"""Reader and writer of the golden vectors under tests/golden/ (make_golden.py, make_train_golden.py,
+make_dropin_golden.py)."""
+import glob
 import os
 from collections import defaultdict
 
@@ -6,17 +8,47 @@ import numpy as np
 import torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+SHARD_BYTES = 900000         # raw bytes per file, per-array zip / .npy headers included: every file stays under 1 MB
 _cache = {}
 
 
+def _shards(fname):
+    stem = os.path.join(GOLDEN, fname[:-len(".npz")])
+    return sorted(glob.glob(stem + ".*.npz"), key=lambda p: int(p.rsplit(".", 2)[1]))
+
+
+def save(fname, arrays):
+    """{"case|group|name": array} -> tests/golden/<stem>.<i>.npz, compressed; arrays go into the shards in order and a
+    shard is closed before its raw size passes SHARD_BYTES."""
+    for old in _shards(fname):
+        os.remove(old)
+    stem = os.path.join(GOLDEN, fname[:-len(".npz")])
+    shards, size = [{}], 0
+    for key, value in arrays.items():
+        value = np.asarray(value)
+        n = value.nbytes + 512
+        if shards[-1] and size + n > SHARD_BYTES:
+            shards.append({})
+            size = 0
+        shards[-1][key] = value
+        size += n
+    for i, shard in enumerate(shards):
+        np.savez_compressed("%s.%d.npz" % (stem, i), **shard)
+    total = sum(os.path.getsize(p) for p in _shards(fname))
+    print("wrote %s: %d arrays in %d files, %.1f KB" % (fname, len(arrays), len(shards), total / 1024))
+
+
 def load(fname):
-    """-> {case: {group: {name: np.ndarray}}}"""
+    """-> {case: {group: {name: np.ndarray}}} of all shards of ``fname``"""
     if fname not in _cache:
-        z = np.load(os.path.join(GOLDEN, fname), allow_pickle=False)
+        paths = _shards(fname)
+        assert paths, "no golden shards for %s under %s" % (fname, GOLDEN)
         out = defaultdict(lambda: defaultdict(dict))
-        for key in z.files:
-            case, group, name = key.split("|")
-            out[case][group][name] = z[key]
+        for path in paths:
+            z = np.load(path, allow_pickle=False)
+            for key in z.files:
+                case, group, name = key.split("|")
+                out[case][group][name] = z[key]
         _cache[fname] = out
     return _cache[fname]
 

@@ -37,7 +37,10 @@ def _check_case(case, outs, sd, inputs):
     grads = _grads(outs, leaves)
     for k, g in zip(names + list(case.get("gin", {})), grads):
         ref = case["gsd"][k] if k in case["gsd"] else case["gin"][k]
-        close(g, ref, rtol=1e-3, atol=2e-4)
+        # fp32 gradient sums carry rounding error in proportion to the tensor's largest entries, and its size depends
+        # on the CPU's kernels: small entries of a large-valued weight gradient get an absolute allowance of 1e-5 of
+        # that scale on top of 2e-4
+        close(g, ref, rtol=1e-3, atol=2e-4 + 1e-5 * float(np.abs(ref).max()))
 
 
 BLOCKS = G.load("blocks.npz")
