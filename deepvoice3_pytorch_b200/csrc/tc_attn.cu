@@ -324,6 +324,9 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attn_rows_kernel(const __grid_c
             }
             r0v = dot;
         }
+        // probability of a masked key: 0, but NaN in a row whose keys are all masked (max -inf), which has no softmax
+        // -- the SIMT kernel and torch's softmax of a row of -inf give NaN there too
+        const float pr_masked = (BWD == 0 && r0v == -INFINITY) ? __int_as_float(0x7fc00000) : 0.f;
         // final pass: produce the row of the second GEMM's A operand (dropout(P) or dS), write P / dS to HBM
         for (int c32 = 0; c32 < AT_NS; c32 += 32) {
             float v[32], o[32];
@@ -345,7 +348,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attn_rows_kernel(const __grid_c
                 if (tv && s < Ts) {
                     if (BWD == 0) {
                         const bool ok = !((mbc >> i) & 1u);
-                        const float pr = ok ? expf(v[i] - r0v) * r1v : 0.f;
+                        const float pr = ok ? expf(v[i] - r0v) * r1v : pr_masked;
                         wr = pr;
                         a2 = pr * drop_scale(drop, (uint32_t)(rbase + s));
                     } else {

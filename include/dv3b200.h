@@ -127,7 +127,10 @@ int dv3_bgemm(const float* A, long long sAb, long long sAm, long long sAk, const
  * null -> probs (B,Td,Ts) = softmax(q^T k) (pre-dropout, returned as the alignment), out (B,E,Td) =
  * scale * v . dropout(probs)^T.  Backward: dout (B,E,Td), dprobs (B,Td,Ts) gradient arriving at the returned
  * probabilities (or null) -> dq, dk, dv; ds is a (B,Td,Ts) scratch.  Shapes: dv3_tc_attn_supported (Ts <= 128,
- * E % 16 == 0, E <= 256); others go through dv3_bgemm + dv3_softmax_*. */
+ * E % 16 == 0, E <= 256); others go through dv3_bgemm + dv3_softmax_*.  An utterance whose keys are all masked has
+ * no softmax: both paths return NaN for its probabilities and context, as torch's softmax of a row of -inf does, and
+ * NaN for its dq, dk and dv (torch's masked_fill backward gives 0 for dq and dk there; the loss is NaN either way).
+ * Pinned by tests/test_gpu_attention_core.py. */
 int dv3_tc_attn_supported(int B, int E, int Td, int Ts);
 int dv3_tc_attn_fwd(const float* q, const float* k, const float* v, const unsigned char* mask, float* probs,
                     float* out, int B, int E, int Td, int Ts, float scale, float p_drop,
