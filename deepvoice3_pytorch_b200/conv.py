@@ -47,12 +47,12 @@ class Conv1d(_WeightNormed):
         b = init_bias if init_bias is not None else torch.zeros(out_channels)
         self._set_params(w, b)
 
-    def forward(self, x, relu=False, causal=None, chain=None, training=False):
+    def forward(self, x, relu=False, causal=None):
         """causal=None: treat causal padding like the reference does (output length T + (k-1)d is not
         produced; callers of the causal form always trim to T, which is what the kernel computes)."""
         causal = self.causal_padding if causal is None else causal
         return ops.conv1d(x, self.weight_v, self.weight_g, self.bias, self.kernel_size[0], self.dilation[0],
-                          causal=causal, relu=relu, chain=chain, training=training)
+                          causal=causal, relu=relu)
 
     def incremental_forward(self, input):
         """input (B, T, Cin): the newest frame input[:, -1] enters the ring buffer of the last (k-1)*dilation+1
@@ -89,8 +89,8 @@ class ConvTranspose1d(_WeightNormed):
         b = init_bias if init_bias is not None else torch.zeros(out_channels)
         self._set_params(w, b)
 
-    def forward(self, x, chain=None):
-        return ops.conv_transpose1d_k2s2(x, self.weight_v, self.weight_g, self.bias, chain=chain)
+    def forward(self, x):
+        return ops.conv_transpose1d_k2s2(x, self.weight_v, self.weight_g, self.bias)
 
 
 class WNLinear(_WeightNormed):

@@ -21,12 +21,6 @@
 // accumulator sets, so the epilogue warps drain tile n while the MMA thread accumulates tile n+1 and the TMA ring
 // streams across tile boundaries.  Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer,
 // warps 2-5 = epilogue (TMEM -> registers -> fused math -> stores coalesced along T).
-//
-// What the epilogues fuse besides the block's own math (Dv3TcFuse, include/dv3b200.h):
-//   * forward: the bf16 hi/lo planes -- with the CONSUMER's input dropout applied -- that the next convolution reads,
-//     so chained blocks need no operand-split pass;
-//   * data gradient: the backward of the PRODUCER of the tensor whose gradient this call computes (GLU / highway gate,
-//     ReLU or identity), emitted as that producer's dAB planes + bias-gradient sums, so no gate-backward pass.
 #include "tc_common.cuh"
 #include "../../include/dv3b200.h"
 
@@ -37,14 +31,10 @@ using namespace tc;
 constexpr int TC_THREADS = 192;
 constexpr int MAX_TAPS_TC = 8;
 constexpr int SMEM_LIMIT = 232448;          // 227 KB opt-in dynamic shared memory per CTA
-constexpr int EPI_BUF = 16384;              // epilogue -> TMA-store staging buffer: hi 8 KB | lo 8 KB
-constexpr int EPI_STAGING = 2 * EPI_BUF;
 
 enum { TC_GATED = 0, TC_CONV = 1 };
-enum { POST_NONE = 0, POST_GLU = 1, POST_HIGHWAY = 2, POST_RELU = 3, POST_IDENT = 4 };
 
-struct TcMaps { CUtensorMap a[2]; CUtensorMap b[2]; CUtensorMap st[4]; };   // st: planes written by the epilogue
-                                                                            // (hi, lo) [+ (hi, lo) of the bf16 copy]
+struct TcMaps { CUtensorMap a[2]; CUtensorMap b[2]; };
 
 struct TcParams {
     int T, B;
@@ -60,13 +50,6 @@ struct TcParams {
     // conv epilogue: out = acc*dropmask + bias + addend ; relu
     float* out; const float* e1; const float* e2; float alpha; int addmode, relu;
     float p_drop; const unsigned long long* seed_ptr; uint32_t salt;
-    // forward fusion: planes of (output * next dropout mask) for the consumer conv, [2][B][T][np_pitch]
-    __nv_bfloat16* np; int np_pitch; long long np_plane; int np_wg;    // np_wg: also emit the bf16 pair (maps.st[2..3])
-    float np_p; const unsigned long long* np_seed; uint32_t np_salt;
-    // backward fusion: producer backward applied to the data gradient this launch computes
-    int post_kind, post_residual, post_pitch;
-    const float* post_a; const float* post_s; const float* post_x;
-    __nv_bfloat16* post_planes; long long post_plane; float* post_dbias;
     // Compensation of the tensor core's truncating accumulation: every tcgen05.mma adds its K = 16 partial product
     // into the fp32 accumulator rounding TOWARD ZERO, an expected relative loss of ~0.35 * 2^-23 per event on the
     // running sum; over the n_mma events of one output that is a systematic shrink of ~gcoef * n_mma (measured,
@@ -96,11 +79,17 @@ struct TcCfg {
     static constexpr int TILE = 128 * BK * 2;            // A tile (128 rows)
     static constexpr int TILE_B = BR * BK * 2;           // one B box
     static constexpr int STAGE = 2 * (TILE + NBOX * TILE_B);
-    static constexpr int STAGES_RAW = (SMEM_LIMIT - 2048 - EPI_STAGING) / STAGE;
+    static constexpr int STAGES_RAW = (SMEM_LIMIT - 2048) / STAGE;
     static constexpr int STAGES = STAGES_RAW > 6 ? 6 : STAGES_RAW;
-    static constexpr int SMEM = STAGES * STAGE + EPI_STAGING + 1024 + 512;   // + alignment slack + barriers
+    static constexpr int SMEM = STAGES * STAGE + 1024 + 512;   // + alignment slack + barriers
     static constexpr int NCOLS = BR * NBOX;              // columns per accumulator; (main, cross) x two sets
 };
+// Ring depths of the instantiations the host code launches (<NBOX, BK, BR>), pinned so a change is deliberate.
+static_assert(TcCfg<2, 64, 64>::STAGES == 3, "gated <0,2,64,64>");
+static_assert(TcCfg<1, 64, 128>::STAGES == 3, "conv <1,1,128,64>");
+static_assert(TcCfg<1, 64, 64>::STAGES == 4, "conv <1,1,64,64>");
+static_assert(TcCfg<1, 32, 128>::STAGES == 6, "conv <1,1,128,32>");
+static_assert(TcCfg<1, 32, 64>::STAGES == 6, "conv <1,1,64,32>");
 
 // main + cross accumulator -> registers, summed in fp32 (round-to-nearest)
 // gmain = 1 + (expected relative truncation loss of the main accumulator), see TcParams::gmain
@@ -112,81 +101,6 @@ __device__ __forceinline__ void tmem_ld_add(uint32_t taddr, int cross_off, float
     for (int i = 0; i < 32; ++i) v[i] = fmaf(c[i], LO_INV, v[i] * gmain);       // lo planes carry a 2^11 scale
 }
 
-// ---- operand planes written by the epilogues: registers -> shared-memory staging -> TMA tensor store ---------------
-// The epilogue thread of accumulator row r (time step) holds 32 consecutive channels; the planes are (B,T,C) with C
-// contiguous, so direct stores would be 16-byte pieces 1-2 KB apart (32 LSU wavefronts per instruction: measured 2.3x
-// slower data-gradient kernels).  Instead the 128 epilogue threads write their rows into a [128][64 B] staging tile
-// (SWIZZLE_64B: conflict-free) and one thread hands the tile to the TMA unit (cp.async.bulk.tensor store), which
-// also clips rows >= T and pad channels.  Two staging buffers alternate; a buffer is rewritten once the bulk group
-// that read it has drained (cp.async.bulk.wait_group.read 1).
-__device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                 ::"l"(map), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-struct EpiStage {
-    uint8_t* base;             // EPI_STAGING bytes, 1024-aligned
-    const CUtensorMap* map;    // [2]: hi, lo
-    int uses;                  // buffer = uses & 1
-    bool issuer;
-};
-
-// One use = one [128 rows][32 channels] tile of one output tensor: FMT_F16 (forward operand) or FMT_BF16 (gradient).
-template <int FMT>
-__device__ __forceinline__ void epi_emit(EpiStage& es, int row, const float* v, int c0, int t0, int b, int map0 = 0) {
-    uint8_t* buf = es.base + (es.uses & 1) * EPI_BUF;
-    __syncwarp();                                        // bar.sync needs converged warps
-    if (es.issuer) bulk_wait_read<1>();                  // the group that last read this buffer has drained
-    __syncwarp();
-    epi_bar();
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        uint32_t h[4], l[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            uint16_t h0, l0, h1, l1;
-            split_pair<FMT>(v[j * 8 + 2 * i], h0, l0);
-            split_pair<FMT>(v[j * 8 + 2 * i + 1], h1, l1);
-            h[i] = (uint32_t)h0 | ((uint32_t)h1 << 16);
-            l[i] = (uint32_t)l0 | ((uint32_t)l1 << 16);
-        }
-        const uint32_t off = (uint32_t)row * 64u + (uint32_t)((j ^ ((row >> 1) & 3)) << 4);   // SWIZZLE_64B
-        *reinterpret_cast<uint4*>(buf + off) = make_uint4(h[0], h[1], h[2], h[3]);
-        *reinterpret_cast<uint4*>(buf + 8192 + off) = make_uint4(l[0], l[1], l[2], l[3]);
-    }
-    fence_proxy_async();
-    __syncwarp();
-    epi_bar();
-    if (es.issuer) {
-        tma_store_3d(&es.map[map0], buf, c0, t0, b);
-        tma_store_3d(&es.map[map0 + 1], buf + 8192, c0, t0, b);
-        bulk_commit();
-    }
-    ++es.uses;
-}
-
-// Column sums over the 32 rows held by the lanes of a warp: after the call lane i holds sum_rows v[i].
-// Butterfly "transpose-reduce": 31 shuffles instead of 32 x 5.
-__device__ __forceinline__ float warp_colsum32(float* v, int lane) {
-#pragma unroll
-    for (int half = 16; half >= 1; half >>= 1) {
-        const bool upper = (lane & half) != 0;
-#pragma unroll
-        for (int i = 0; i < half; ++i) {
-            // lanes with the bit set keep columns [half, 2*half), the others [0, half); exchange the other part
-            const float send = upper ? v[i] : v[i + half];
-            const float recv = __shfl_xor_sync(0xffffffffu, send, half);
-            v[i] = (upper ? v[i + half] : v[i]) + recv;
-        }
-    }
-    return v[0];
-}
-
 // ---- epilogues -----------------------------------------------------------------------------------------------
 // NOTE on the epilogue loads: residual / addend / bias reads go through __ldg (ld.global.nc) and are issued as a
 // batch of 32 independent loads BEFORE the dependent math and stores of the chunk.  With plain loads the compiler
@@ -194,7 +108,7 @@ __device__ __forceinline__ float warp_colsum32(float* v, int lane) {
 // global-memory round trips per thread (ncu: 40 % of the stall samples sat on the first use of these loads).
 template <int BR, int NCOLS>
 __device__ __forceinline__ void epilogue_gated(const TcParams& p, uint32_t taddr, int a_row0, int a_z, int b_row0,
-                                               int row, EpiStage& es) {
+                                               int row) {
     const int t = a_row0 + row, b = a_z, C = p.Nc;
     const bool tv = t < p.T;
     const float* __restrict__ bias = p.bias;
@@ -205,7 +119,6 @@ __device__ __forceinline__ void epilogue_gated(const TcParams& p, uint32_t taddr
     float* __restrict__ so = p.save_s;
     const bool need_res = (p.gate_mode != 0) || p.residual;
     const size_t base = ((size_t)b * C + b_row0) * p.T + (tv ? t : 0);
-    const DropCfg nd = make_drop(p.np ? p.np_p : 0.f, p.np_seed, p.np_salt);
     for (int c32 = 0; c32 < BR; c32 += 32) {
         float va[32], vb[32], rr[32];
         tmem_ld_add(taddr + c32, NCOLS, va, p.gmain);
@@ -234,33 +147,21 @@ __device__ __forceinline__ void epilogue_gated(const TcParams& p, uint32_t taddr
                 yo[idx] = y;
                 if (ao) ao[idx] = a;
                 if (so) so[idx] = s;
-                va[i] = y * drop_scale(nd, (uint32_t)idx);          // the consumer's conv-input dropout
             }
-        }
-        // all 128 epilogue threads reach the emission together (named barriers inside); rows >= T are clipped by TMA
-        if (p.np) {
-            epi_emit<FMT_F16>(es, row, va, b_row0 + c32, a_row0, b);
-            if (p.np_wg) epi_emit<FMT_BF16>(es, row, va, b_row0 + c32, a_row0, b, 2);
         }
     }
 }
 
 template <int NCOLS>
 __device__ __forceinline__ void epilogue_conv(const TcParams& p, uint32_t taddr, int a_row0, int a_z, int b_row0,
-                                              int row, int lane, EpiStage& es) {
+                                              int row) {
     const int t = a_row0 + row, b = a_z;
     const bool tv = t < p.T;
     const DropCfg drop = make_drop(p.p_drop, p.seed_ptr, p.salt);
-    const DropCfg nd = make_drop(p.np ? p.np_p : 0.f, p.np_seed, p.np_salt);
     const float* __restrict__ bias = p.bias;
     const float* __restrict__ e1 = p.e1;
     const float* __restrict__ e2 = p.e2;
-    const float* __restrict__ pa = p.post_a;
-    const float* __restrict__ ps = p.post_s;
-    const float* __restrict__ px = p.post_x;
     float* __restrict__ out = p.out;
-    const int kind = p.post_kind;
-    const float gs = (kind == POST_GLU && p.post_residual) ? 0.70710678118654752f : 1.f;
     for (int c32 = 0; c32 < NCOLS; c32 += 32) {
         float v[32], x1[32], x2[32];
         tmem_ld_add(taddr + c32, NCOLS, v, p.gmain);
@@ -276,66 +177,15 @@ __device__ __forceinline__ void epilogue_conv(const TcParams& p, uint32_t taddr,
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
                 const int n = n0 + i;
-                float g = 0.f;
                 if (n < p.Nc) {
                     const size_t idx = cb + (size_t)i * p.T;
-                    g = v[i] * drop_scale(drop, (uint32_t)idx);
+                    float g = v[i] * drop_scale(drop, (uint32_t)idx);
                     if (bias) g += __ldg(&bias[n]);
                     if (p.addmode == 1) g += p.alpha * x1[i];
                     else if (p.addmode == 2) g += x1[i] * (1.f - x2[i]);
                     if (p.relu) g = fmaxf(g, 0.f);
                     out[idx] = g;
                 }
-                v[i] = g;
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = 0.f;
-        }
-        if (p.np) {                                         // forward: operand planes of the consumer
-            float w[32];
-#pragma unroll
-            for (int i = 0; i < 32; ++i) w[i] = v[i] * drop_scale(nd, (uint32_t)(cb + (size_t)i * p.T));
-            epi_emit<FMT_F16>(es, row, w, n0, a_row0, b);
-            if (p.np_wg) epi_emit<FMT_BF16>(es, row, w, n0, a_row0, b, 2);
-        }
-        if (kind != POST_NONE) {                            // backward of the producer of this gradient's tensor
-            // v[i] = dL/d(producer output) at (b, n0+i, t) (0 outside the tile).  Gate kinds emit [da | db] planes of
-            // width 2*Nc, the others a single gradient plane of width post_pitch.
-            float da[32], db[32];
-            if (kind == POST_GLU || kind == POST_HIGHWAY) {
-#pragma unroll
-                for (int i = 0; i < 32; ++i) {
-                    float av = 0.f, sv = 0.f, xv = 0.f;
-                    if (tv && n0 + i < p.Nc) {
-                        const size_t idx = cb + (size_t)i * p.T;
-                        av = __ldg(&pa[idx]); sv = __ldg(&ps[idx]);
-                        if (kind == POST_HIGHWAY) xv = __ldg(&px[idx]);
-                    }
-                    const float g = v[i] * gs;
-                    da[i] = g * sv;
-                    db[i] = g * (kind == POST_GLU ? av : (av - xv)) * sv * (1.f - sv);
-                }
-                epi_emit<FMT_BF16>(es, row, da, n0, a_row0, b);
-                epi_emit<FMT_BF16>(es, row, db, p.Nc + n0, a_row0, b);
-                const float sa = warp_colsum32(da, lane), sb = warp_colsum32(db, lane);
-                if (p.post_dbias && n0 + lane < p.Nc) {
-                    atomicAdd(&p.post_dbias[n0 + lane], sa);
-                    atomicAdd(&p.post_dbias[p.Nc + n0 + lane], sb);
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < 32; ++i) {
-                    float g = v[i];
-                    if (kind == POST_RELU) {
-                        const bool on = tv && n0 + i < p.Nc && __ldg(&pa[cb + (size_t)i * p.T]) > 0.f;
-                        g = on ? g : 0.f;
-                    }
-                    da[i] = g;
-                }
-                epi_emit<FMT_BF16>(es, row, da, n0, a_row0, b);
-                const float sa = warp_colsum32(da, lane);
-                if (p.post_dbias && n0 + lane < p.Nc) atomicAdd(&p.post_dbias[n0 + lane], sa);
             }
         }
     }
@@ -356,8 +206,7 @@ tc_conv_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
     static_assert(STAGES >= 2, "pipeline needs at least two stages");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint8_t* staging = smem + STAGES * STAGE;                // epilogue -> TMA store tiles (1024-aligned: STAGE % 1024 == 0)
-    uint64_t* full = reinterpret_cast<uint64_t*>(staging + EPI_STAGING);
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + STAGES * STAGE);
     uint64_t* empty = full + STAGES;
     uint64_t* tfull = empty + STAGES;          // [2] accumulator set ready for the epilogue
     uint64_t* tempty = tfull + 2;              // [2] accumulator set drained
@@ -367,8 +216,6 @@ tc_conv_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
 
     if (threadIdx.x == 0) {
         prefetch_tmap(&maps.a[0]); prefetch_tmap(&maps.a[1]); prefetch_tmap(&maps.b[0]); prefetch_tmap(&maps.b[1]);
-        if (p.np || p.post_kind) { prefetch_tmap(&maps.st[0]); prefetch_tmap(&maps.st[1]); }
-        if (p.np_wg) { prefetch_tmap(&maps.st[2]); prefetch_tmap(&maps.st[3]); }
         for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
         for (int a = 0; a < 2; ++a) { mbar_init(&tfull[a], 1); mbar_init(&tempty[a], 128); }
         fence_barrier_init();
@@ -440,8 +287,6 @@ tc_conv_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
         }
     } else if (warp >= 2) {
         const int q = warp & 3, row = q * 32 + lane;
-        EpiStage es;
-        es.base = staging; es.map = maps.st; es.uses = 0; es.issuer = (warp == 2 && lane == 0);
         int tcount = 0;
         for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++tcount) {
             int a_row0, a_z, b_row0, b_row1;
@@ -450,12 +295,11 @@ tc_conv_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
             mbar_wait(&tfull[a], aph);
             tc_fence_after();
             const uint32_t taddr = tmem_base + a * 2 * NCOLS + ((uint32_t)(q * 32) << 16);
-            if (MODE == TC_GATED) epilogue_gated<BR, NCOLS>(p, taddr, a_row0, a_z, b_row0, row, es);
-            else epilogue_conv<NCOLS>(p, taddr, a_row0, a_z, b_row0, row, lane, es);
+            if (MODE == TC_GATED) epilogue_gated<BR, NCOLS>(p, taddr, a_row0, a_z, b_row0, row);
+            else epilogue_conv<NCOLS>(p, taddr, a_row0, a_z, b_row0, row);
             tc_fence_before();
             mbar_arrive(&tempty[a]);                                // 128 arrivals release the set to the MMA thread
         }
-        if (es.issuer) bulk_wait_all();                             // plane stores complete before the CTA exits
     }
     tc_fence_before();
     __syncthreads();
@@ -694,51 +538,12 @@ int dv3_tc_conv_supported(int B, int Cin, int Cout, int T, int k) {
            Cout >= 1;
 }
 
-// planes written by the epilogue: [2][B][T][pitch], stored as [128 rows][32 channels] boxes (SWIZZLE_64B staging)
-static int encode_store_maps(TcMaps& maps, int first, void* planes, int pitch, int B, int T) {
-    for (int pl = 0; pl < 2; ++pl)
-        if (encode_tmap_bf16_3d(&maps.st[first + pl], plane(planes, pl, (long long)B * T * pitch), pitch, T, B,
-                                (uint64_t)pitch * 2, (uint64_t)T * pitch * 2, 32, 128)) return 1;
-    return 0;
-}
-
-static int apply_fuse(TcParams& p, TcMaps& maps, const Dv3TcFuse* f, int B, int T, int out_channels, const char* what) {
-    if (!f) return 0;
-    DV3_REQUIRE(!(f->np && f->post_kind != POST_NONE), "%s: np and post_kind are exclusive (forward vs data gradient)", what);
-    if (f->np) {
-        DV3_REQUIRE(f->np_pitch >= out_channels && f->np_pitch % 8 == 0, "%s: np_pitch %d must be pad8 of %d channels",
-                    what, f->np_pitch, out_channels);
-        p.np = (__nv_bfloat16*)f->np; p.np_pitch = f->np_pitch; p.np_plane = (long long)B * T * f->np_pitch;
-        p.np_p = f->np_p; p.np_seed = f->np_seed; p.np_salt = f->np_salt;
-        if (encode_store_maps(maps, 0, f->np, f->np_pitch, B, T)) return 1;
-        if (f->np_wg) {
-            p.np_wg = 1;
-            if (encode_store_maps(maps, 2, f->np_wg, f->np_pitch, B, T)) return 1;
-        }
-    }
-    if (f->post_kind != POST_NONE) {
-        DV3_REQUIRE(f->post_kind >= POST_GLU && f->post_kind <= POST_IDENT && f->post_planes, "%s: bad post_kind %d",
-                    what, f->post_kind);
-        const bool gate = f->post_kind == POST_GLU || f->post_kind == POST_HIGHWAY;
-        DV3_REQUIRE(!gate || (f->post_a && f->post_s && out_channels % 8 == 0), "%s: gate backward needs saved a, s", what);
-        DV3_REQUIRE(f->post_kind != POST_HIGHWAY || f->post_x, "%s: highway backward needs the block input", what);
-        DV3_REQUIRE(f->post_kind != POST_RELU || f->post_a, "%s: ReLU backward needs the producer output", what);
-        p.post_kind = f->post_kind; p.post_residual = f->post_residual;
-        p.post_a = f->post_a; p.post_s = f->post_s; p.post_x = f->post_x;
-        p.post_planes = (__nv_bfloat16*)f->post_planes;
-        p.post_pitch = gate ? 2 * out_channels : (out_channels + 7) / 8 * 8;
-        p.post_plane = (long long)B * T * p.post_pitch;
-        p.post_dbias = f->post_dbias;
-        if (encode_store_maps(maps, 0, f->post_planes, p.post_pitch, B, T)) return 1;
-    }
-    return 0;
-}
-
 // Gated forward.  xd: [2][B][T][C] bf16 planes of the (dropped-out) input; w: [2][k][2C][C] bf16 planes of the
 // normalised weight; the rest as dv3_convblock_fwd.  64-channel tiles (64 a | 64 b columns), BK = 64.
 int dv3_tc_convblock_fwd(const void* xd, const void* w, int npl, const float* bias, const float* spk,
                          const float* res, float* y, float* save_a, float* save_s, int B, int C, int T, int k,
-                         int dilation, int causal, int mode, int residual, const Dv3TcFuse* fuse, void* stream) {
+                         int dilation, int causal, int mode, int residual, const void* reserved, void* stream) {
+    DV3_REQUIRE(reserved == nullptr, "tc_convblock_fwd: reserved must be NULL");
     DV3_REQUIRE(dv3_tc_supported(B, C, T, k), "tc_convblock_fwd: unsupported shape B=%d C=%d T=%d k=%d", B, C, T, k);
     DV3_REQUIRE(npl == 2, "tc_convblock_fwd: npl must be 2");
     TcMaps maps;
@@ -756,8 +561,6 @@ int dv3_tc_convblock_fwd(const void* xd, const void* w, int npl, const float* bi
     p.gate_mode = mode; p.residual = residual;
     p.gmain = 1.f + config().tc_gamma * (float)(p.k * p.kb_n * 4);
     p.idesc_fmt = IDESC_A_F16 | IDESC_B_F16;                     // forward operands: fp16 hi/lo planes
-    if (apply_fuse(p, maps, fuse, B, T, C, "tc_convblock_fwd")) return 1;
-    DV3_REQUIRE(p.post_kind == POST_NONE, "tc_convblock_fwd: post_kind is a data-gradient option");
     return launch_conv<TC_GATED, 2, 64, 64>(maps, p, t_tiles, C / 64, B, (cudaStream_t)stream, "tc_convblock_fwd");
 }
 
@@ -769,7 +572,8 @@ int dv3_tc_convblock_fwd(const void* xd, const void* w, int npl, const float* bi
 int dv3_tc_conv(const void* a, const void* w, int npl, float* out, int B, int Kc, int Nc, int T, int k, int dilation,
                 int causal, int transpose_taps, const float* bias, int relu, float p_drop,
                 const unsigned long long* seed_ptr, unsigned salt, int addmode, const float* e1, const float* e2,
-                float alpha, const Dv3TcFuse* fuse, void* stream) {
+                float alpha, const void* reserved, void* stream) {
+    DV3_REQUIRE(reserved == nullptr, "tc_conv: reserved must be NULL");
     DV3_REQUIRE(k >= 1 && k <= MAX_TAPS_TC && (k == 1 || Nc % 128 == 0) && B <= 65535,
                 "tc_conv: unsupported shape B=%d Kc=%d Nc=%d T=%d k=%d", B, Kc, Nc, T, k);
     DV3_REQUIRE(npl == 2, "tc_conv: npl must be 2");
@@ -795,7 +599,6 @@ int dv3_tc_conv(const void* a, const void* w, int npl, float* out, int B, int Kc
     p.gmain = 1.f + config().tc_gamma * (float)(p.k * p.kb_n * (bk / 16));
     // forward conv: fp16 activation x fp16 weight planes; data gradient: bf16 gradient x bf16 weight planes
     p.idesc_fmt = transpose_taps ? (IDESC_A_BF16 | IDESC_B_BF16) : (IDESC_A_F16 | IDESC_B_F16);
-    if (apply_fuse(p, maps, fuse, B, T, Nc, "tc_conv")) return 1;
     const int tiles_y = (Nc + br - 1) / br;
     if (narrow) {
         if (k64) return launch_conv<TC_CONV, 1, 64, 64>(maps, p, t_tiles, tiles_y, B, st, "tc_conv(64)");

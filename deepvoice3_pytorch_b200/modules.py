@@ -139,9 +139,8 @@ class Conv1dGLU(_GatedConv):
         self._make_conv(in_channels, out_channels, kernel_size, padding, dilation, causal, dropout, std_mul)
         self.speaker_proj = Linear(speaker_embed_dim, out_channels) if n_speakers > 1 else None
 
-    def forward(self, x, speaker_embed=None, fuse_residual=None, chain=None):
+    def forward(self, x, speaker_embed=None, fuse_residual=None):
         """x (B, C, T); speaker_embed (B, T, S) time-expanded (and, in training, dropped-out) embedding.
-        chain: ops.Chain from run_conv_stack (what the kernel epilogues may fuse with the neighbouring layers).
         fuse_residual=True computes (block(x) + x)*sqrt(.5) in the kernel even when the module was built with
         residual=False -- the decoder applies exactly that outside the block when no attention layer sits in between
         (reference deepvoice3.py:333-349)."""
@@ -151,7 +150,7 @@ class Conv1dGLU(_GatedConv):
         c = self.conv
         residual = self.residual if fuse_residual is None else bool(fuse_residual)
         return ops.convblock(x, c.weight_v, c.weight_g, c.bias, spk, c.kernel_size[0], c.dilation[0],
-                             self.causal, ops.MODE_GLU, residual, self.dropout, self.training, chain=chain)
+                             self.causal, ops.MODE_GLU, residual, self.dropout, self.training)
 
 
     def incremental_forward(self, x, speaker_embed=None):
@@ -176,10 +175,10 @@ class HighwayConv1d(_GatedConv):
         self._make_conv(in_channels, out_channels, kernel_size, padding, dilation, causal, dropout,
                         1.0 if std_mul is None else std_mul)
 
-    def forward(self, x, chain=None):
+    def forward(self, x):
         c = self.conv
         return ops.convblock(x, c.weight_v, c.weight_g, c.bias, None, c.kernel_size[0], c.dilation[0],
-                             self.causal, ops.MODE_HIGHWAY, True, self.dropout, self.training, chain=chain)
+                             self.causal, ops.MODE_HIGHWAY, True, self.dropout, self.training)
 
     def incremental_forward(self, x):
         """reference modules.py:197-198."""
@@ -200,47 +199,25 @@ def get_mask_from_lengths(memory, memory_lengths):
     return (~mask).to(memory.device)
 
 
-def _consumer_dropout(f):
-    """Input dropout the next layer applies to its conv input, or None when it is not a conv whose operand planes /
-    producer backward the previous layer's epilogue can prepare."""
-    if isinstance(f, (Conv1dGLU, HighwayConv1d)):
-        return float(f.dropout)
-    if isinstance(f, (_Conv1d, _ConvTranspose1d)):
-        return 0.0
-    return None
-
-
 def run_conv_stack(layers, x, speaker_embed_btc=None, boundaries=None):
     """Run a ModuleList/Sequential of [Conv1d | ReLU | Sigmoid | ConvTranspose1d | Conv1dGLU | HighwayConv1d]
-    on x (B, C, T), fusing every ``Conv1d -> ReLU`` pair into one kernel launch.  Inside the stack every tensor has
-    exactly one consumer -- the next layer -- which is what lets the tensor-core epilogues prepare the next layer's
-    operand planes (forward) and run the previous layer's gate / ReLU backward (data gradient): ops.Chain.
+    on x (B, C, T), fusing every ``Conv1d -> ReLU`` pair into one kernel launch.
     boundaries: {layer index: tag} -- the input of that layer is an ops.grad_boundary (its gradient being ready means
     the parameter gradients of layers[index:] are final)."""
     layers = list(layers)
-    i, follows = 0, False
+    i = 0
     while i < len(layers):
         f = layers[i]
         if boundaries and i in boundaries:
             x = ops.grad_boundary(x, boundaries[i])
         fuse_relu = isinstance(f, _Conv1d) and i + 1 < len(layers) and isinstance(layers[i + 1], nn.ReLU)
-        nxt = i + (2 if fuse_relu else 1)
-        emit_p = _consumer_dropout(layers[nxt]) if nxt < len(layers) else None
-        chain = ops.Chain(follows, emit_p, emit_p is not None)
-        follows = True
         if isinstance(f, _Conv1d):
-            x = f(x, relu=fuse_relu, chain=chain, training=f.training)
+            x = f(x, relu=fuse_relu)
         elif isinstance(f, Conv1dGLU):
-            x = f(x, speaker_embed_btc, chain=chain)
-        elif isinstance(f, HighwayConv1d):
-            x = f(x, chain=chain)
-        elif isinstance(f, _ConvTranspose1d):
-            x = f(x, chain=chain)
+            x = f(x, speaker_embed_btc)
         elif isinstance(f, nn.ReLU):
             x = torch.relu(x)
-            follows = False
         else:
             x = f(x)
-            follows = False
-        i = nxt
+        i += 2 if fuse_relu else 1
     return x

@@ -309,122 +309,11 @@ def _pad8(n):
     return (n + 7) // 8 * 8
 
 
-# ----------------------------------------------------------------------------------------------
-# epilogue fusion between neighbouring convolutions (csrc/tc_gemm.cu, Dv3TcFuse in include/dv3b200.h)
-# ----------------------------------------------------------------------------------------------
-# fuse_fwd: a producer conv writes, from its epilogue, the bf16 operand planes (consumer's input dropout applied) that
-#           the next conv reads -> no dv3_tc_split_input pass between chained blocks.
-# fuse_bwd: the data-gradient GEMM of the consumer applies the producer's backward (gate / ReLU) in its epilogue and
-#           emits the producer's gradient planes + bias-gradient sums -> no dv3_tc_gate_bwd_split / dv3_tc_grad_split.
-# Both need the caller (modules.run_conv_stack) to state that the tensor has exactly ONE consumer.
-# Both are OFF by default: measured on the B200 (profiles/r02_fusion_ab.txt) the fused step is SLOWER (7.26 vs 6.34 ms,
-# forward fusion alone 6.45): the separate split / gate-backward kernels stream at HBM speed with full occupancy, while
-# inside the GEMM the same work is done by the 4 epilogue warps of each SM (latency bound), and at C = 256 the fused
-# data-gradient epilogue of a 128x128 tile takes longer than the tile's MMAs.  Kept opt-in because the arithmetic is
-# bit-identical (tests/test_gpu_fusion.py) and the trade flips for wider layers.
-fuse_fwd = os.environ.get("DV3_FUSE_FWD", "0") == "1"
-fuse_bwd = os.environ.get("DV3_FUSE_BWD", "0") == "1"
-
-POST_GLU, POST_HIGHWAY, POST_RELU, POST_IDENT = 1, 2, 3, 4
-
-
-class Dv3TcFuse(ctypes.Structure):
-    _fields_ = [("np", ctypes.c_void_p), ("np_wg", ctypes.c_void_p), ("np_seed", ctypes.c_void_p), ("np_p", ctypes.c_float),
-                ("np_salt", ctypes.c_uint), ("np_pitch", ctypes.c_int), ("post_kind", ctypes.c_int),
-                ("post_residual", ctypes.c_int), ("post_a", ctypes.c_void_p), ("post_s", ctypes.c_void_p),
-                ("post_x", ctypes.c_void_p), ("post_planes", ctypes.c_void_p), ("post_dbias", ctypes.c_void_p)]
-
-
-class Planes:
-    """Operand planes of (tensor * dropout mask(p, seed, salt)) written by the producer's epilogue:
-    t = [2][B][T][pad8(C)] fp16 pair (forward GEMM operand), wg = the same values as a bf16 pair (weight-gradient
-    operand; None when the producer was told the consumer needs no backward)."""
-
-    def __init__(self, t, wg, C, p, seed_t, salt):
-        self.t, self.wg, self.C, self.p, self.seed_t, self.salt = t, wg, C, p, seed_t, salt
-
-
-class ProducerRec:
-    """What the consumer's data-gradient epilogue needs to run the producer's backward, and where it leaves the
-    result.  kind: POST_*; a, s, x: the producer's saved tensors (a = its output y for POST_RELU); dbias: the buffer
-    the bias-gradient sums are accumulated into (zeroed by the producer's forward bookkeeping below)."""
-
-    def __init__(self, kind, C, residual=False, a=None, s=None, x=None):
-        self.kind, self.C, self.residual, self.a, self.s, self.x = kind, C, residual, a, s, x
-        self.planes = None          # [2][B][T][pitch] gradient planes of the producer, filled by the consumer
-        self.dbias = None
-        self.fused = False
-
-
-def _fuse_struct(emit=None, rec=None, dbias=None):
-    """-> (ctypes pointer | None, keep-alive) for a dv3_tc_* call."""
-    if emit is None and rec is None:
-        return None, None
-    f = Dv3TcFuse()
-    if emit is not None:
-        f.np, f.np_seed, f.np_p, f.np_salt = emit.t.data_ptr(), (emit.seed_t.data_ptr() if emit.seed_t is not None else None), \
-            emit.p, emit.salt
-        f.np_wg = emit.wg.data_ptr() if emit.wg is not None else None
-        f.np_pitch = emit.t.shape[-1]
-    if rec is not None:
-        f.post_kind, f.post_residual = rec.kind, int(rec.residual)
-        f.post_a = rec.a.data_ptr() if rec.a is not None else None
-        f.post_s = rec.s.data_ptr() if rec.s is not None else None
-        f.post_x = rec.x.data_ptr() if rec.x is not None else None
-        f.post_planes = rec.planes.data_ptr()
-        f.post_dbias = dbias.data_ptr() if dbias is not None else None
-    return ctypes.byref(f), f
-
-
-def _new_planes(emit_p, training, B, T, C, dev, need_wg):
-    """Planes buffer + dropout identity for a consumer with input dropout ``emit_p`` (None: nothing to emit).
-    need_wg: also the bf16 pair the consumer's weight gradient reads (the producer passes its own need-backward flag:
-    grad mode is off inside autograd.Function.forward, so it cannot be asked here)."""
-    if emit_p is None or not fuse_fwd:
-        return None
-    p, seed_t, salt = _drop_args(emit_p, training, dev)
-    wg = torch.empty(2, B, T, _pad8(C), device=dev, dtype=torch.bfloat16) if need_wg else None
-    return Planes(torch.empty(2, B, T, _pad8(C), device=dev, dtype=torch.float16), wg, C, p, seed_t, salt)
-
-
-def _usable(xh, C, B, T, p_needed):
-    """A producer-written Planes object matches what this consumer would have split itself."""
-    return (xh is not None and xh.C == C and tuple(xh.t.shape) == (2, B, T, _pad8(C)) and
-            (xh.p > 0.0) == (p_needed > 0.0) and (xh.p == 0.0 or abs(xh.p - p_needed) < 1e-12))
-
-
-def _post_dgrad(rec, sinkable_bias, B, T, dev):
-    """Prepare the consumer-side fusion of producer ``rec``'s backward: allocate its gradient planes and pick the
-    bias-gradient destination.  -> dbias tensor handed to the kernel."""
-    gate = rec.kind in (POST_GLU, POST_HIGHWAY)
-    pitch = 2 * rec.C if gate else _pad8(rec.C)
-    rec.planes = torch.empty(2, B, T, pitch, device=dev, dtype=torch.bfloat16)
-    nb = 2 * rec.C if gate else rec.C
-    if sinkable_bias is not None:
-        dbias = sinkable_bias                       # the producer's bias.grad view in the flat arena: accumulate in place
-        rec.dbias = None
-    else:
-        dbias = rec.dbias = torch.zeros(nb, device=dev)
-    rec.fused = True
-    return dbias
-
-
-def _rec_sink_bias(rec):
-    """The .grad view to accumulate the producer's bias gradient into (gradient sink on), else None."""
-    b = getattr(rec, "bias_param", None)
-    if grad_sink and b is not None and b.grad is not None and b.grad.is_contiguous():
-        return b.grad
-    return None
-
-
 class _ConvBlockTCFn(torch.autograd.Function):
-    """Same contract as _ConvBlockFn on the tcgen05 path: operands are bf16 hi/lo planes.
-    xh: Planes of x written by the producer (or None -> split here); emit_p: input dropout of the single consumer
-    (None: no planes emitted); link: ProducerRec of x's producer when this block is its only consumer."""
+    """Same contract as _ConvBlockFn on the tcgen05 path: operands are bf16 hi/lo planes."""
 
     @staticmethod
-    def forward(ctx, x, v, g, bias, spk, k, dilation, causal, mode, residual, p_drop, training, xh, emit_p, link,
-                want_rec, box):
+    def forward(ctx, x, v, g, bias, spk, k, dilation, causal, mode, residual, p_drop, training):
         _chk(x, v, g, bias, spk)
         B, C, T = x.shape
         dev = x.device
@@ -438,19 +327,9 @@ class _ConvBlockTCFn(torch.autograd.Function):
             scale = torch.empty_like(inv)
             wfwd = torch.empty(2, k, 2 * C, C, device=dev, dtype=torch.float16)
             wbwd = torch.empty(2, k, C, 2 * C, device=dev, dtype=bf)
-        p_eff = float(p_drop) if (training and p_drop > 0.0) else 0.0
-        usable = _usable(xh, C, B, T, p_eff)
-        if usable:                                       # the producer drew our dropout identity (salt order unchanged)
-            p, seed_t, salt = xh.p, xh.seed_t, xh.salt
-        else:
-            p, seed_t, salt = _drop_args(p_drop, training, dev)
-        if usable and (xh.wg is not None or not need_bwd):
-            x_btc, x_wg = xh.t, xh.wg                    # ... and already applied it to the planes it wrote
-            split = False
-        else:
-            x_btc = torch.empty(2, B, T, C, device=dev, dtype=torch.float16)        # forward operand (fp16 pair)
-            x_wg = torch.empty(2, B, T, C, device=dev, dtype=bf) if need_bwd else None  # weight-gradient operand
-            split = True
+        p, seed_t, salt = _drop_args(p_drop, training, dev)
+        x_btc = torch.empty(2, B, T, C, device=dev, dtype=torch.float16)        # forward operand (fp16 pair)
+        x_wg = torch.empty(2, B, T, C, device=dev, dtype=bf) if need_bwd else None  # weight-gradient operand
         seed_ptr = _p(seed_t)
         y = torch.empty_like(x)
         a = torch.empty_like(x) if need_bwd else None
@@ -461,29 +340,18 @@ class _ConvBlockTCFn(torch.autograd.Function):
             with side:                    # weight norm + split depends only on the parameters: overlap it with
                 lib.call("dv3_tc_weightnorm_fwd", _p(v), _p(g), _p(inv), _p(scale), _p(wfwd), 2, _p(wbwd), 2 * C, C,
                          k, _stream())    # the activation split below
-        if split:
-            lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, C, T, k, dilation, int(causal), p,
-                     seed_ptr, salt, _stream())
+        lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, C, T, k, dilation, int(causal), p,
+                 seed_ptr, salt, _stream())
         if side is not None:
             side.join()
-        emit = _new_planes(emit_p, training, B, T, C, dev, need_bwd)
-        fptr, _keep = _fuse_struct(emit=emit)
         lib.call("dv3_tc_convblock_fwd", _p(x_btc), _p(wfwd), 2, _p(bias), _p(spk), _p(x), _p(y), _p(a), _p(s),
-                 B, C, T, k, dilation, int(causal), mode, int(residual), fptr, _stream())
-        rec = None
+                 B, C, T, k, dilation, int(causal), mode, int(residual), None, _stream())
         if need_bwd:
             ctx.save_for_backward(x, v, g, a, s, x_wg, wbwd, inv)
             ctx.cfg = (k, dilation, causal, mode, residual, p, salt, spk is not None, dev)
             ctx.seed_t = seed_t
             ctx.bias_param = bias if bias.is_leaf else None
             ctx.bank = bank
-            ctx.link = link if (fuse_bwd and link is not None and link.C == C) else None
-            if want_rec and fuse_bwd:
-                rec = ProducerRec(POST_GLU if mode == MODE_GLU else POST_HIGHWAY, C, residual, a, s,
-                                  x if mode == MODE_HIGHWAY else None)
-                rec.bias_param = ctx.bias_param
-            ctx.rec = rec
-        box.append((emit, rec))
         return y
 
     @staticmethod
@@ -495,19 +363,10 @@ class _ConvBlockTCFn(torch.autograd.Function):
         B, C, T = x.shape
         bf = torch.bfloat16
         sink = _sink(v, g, ctx.bias_param) if ctx.bias_param is not None else None
-        rec = ctx.rec
-        if rec is not None and rec.fused:
-            # the consumer's data-gradient epilogue already ran this block's gate backward on dy
-            d_btc = rec.planes
-            dbias = None if rec.dbias is None else rec.dbias
-            if sink and dbias is not None:
-                sink[2].add_(dbias)
-            rec.planes = rec.a = rec.s = rec.x = None
-        else:
-            d_btc = torch.empty(2, B, T, 2 * C, device=dev, dtype=bf)
-            dbias = sink[2] if sink else torch.zeros(2 * C, device=dev)
-            lib.call("dv3_tc_gate_bwd_split", _p(dy), _p(a), _p(s), _p(x), _p(d_btc), None, _p(dbias), B, C, T,
-                     mode, int(residual), _stream())
+        d_btc = torch.empty(2, B, T, 2 * C, device=dev, dtype=bf)
+        dbias = sink[2] if sink else torch.zeros(2 * C, device=dev)
+        lib.call("dv3_tc_gate_bwd_split", _p(dy), _p(a), _p(s), _p(x), _p(d_btc), None, _p(dbias), B, C, T,
+                 mode, int(residual), _stream())
         need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
         dv = dg = partials = None
         if need_w:                                   # allocate on the main stream, compute on the side stream
@@ -535,30 +394,23 @@ class _ConvBlockTCFn(torch.autograd.Function):
                 addmode, e1, e2, alpha = (1, dy, None, 0.7071067811865476) if residual else (0, None, None, 0.0)
             else:
                 addmode, e1, e2, alpha = 2, dy, s, 0.0
-            fptr = _keep = None
-            link = ctx.link
-            if link is not None and not link.fused and link.a is not None:
-                pd = _post_dgrad(link, _rec_sink_bias(link), B, T, dev)
-                fptr, _keep = _fuse_struct(rec=link, dbias=pd)
             lib.call("dv3_tc_conv", _p(d_btc), _p(wbwd), 2, _p(dx), B, 2 * C, C, T, k, dilation, int(causal), 1,
-                     None, 0, p, seed_ptr, salt, addmode, _p(e1), _p(e2), alpha, fptr, _stream())
+                     None, 0, p, seed_ptr, salt, addmode, _p(e1), _p(e2), alpha, None, _stream())
         if need_w:
             side.join()
         if sink:                                     # already accumulated into the .grad arena views
             dv = dg = dbias = None
-        elif dbias is None:
-            dbias = torch.zeros(2 * C, device=dev)
         dspk = None
         if has_spk and ctx.needs_input_grad[4]:     # d_a = hi + lo * 2^-11 of the (B,T,2C) planes, back to (B,C,T)
             dspk = transpose12((d_btc[0, :, :, :C].float() + d_btc[1, :, :, :C].float() * (1.0 / 2048.0)).contiguous())
-        return (dx, dv, dg, dbias, dspk) + (None,) * 12
+        return (dx, dv, dg, dbias, dspk) + (None,) * 7
 
 
 class _Conv1dTCFn(torch.autograd.Function):
     """Plain weight-normed conv (+ReLU) on the tcgen05 path (1x1 convs, projections)."""
 
     @staticmethod
-    def forward(ctx, x, v, g, bias, k, dilation, causal, relu, xh, emit_p, training, link, want_rec, box):
+    def forward(ctx, x, v, g, bias, k, dilation, causal, relu):
         _chk(x, v, g, bias)
         B, Cin, T = x.shape
         Cout = v.shape[0]
@@ -574,12 +426,8 @@ class _Conv1dTCFn(torch.autograd.Function):
             wfwd = torch.empty(2, k, Cout, Cinp, device=dev, dtype=torch.float16)
             wbwd = torch.empty(2, k, Cin, Coutp, device=dev, dtype=bf)
         need_w = need_bwd and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
-        split = not (_usable(xh, Cin, B, T, 0.0) and (xh.wg is not None or not need_w))
-        if split:
-            x_btc = torch.empty(2, B, T, Cinp, device=dev, dtype=torch.float16)
-            x_wg = torch.empty(2, B, T, Cinp, device=dev, dtype=bf) if need_w else None
-        else:
-            x_btc, x_wg = xh.t, xh.wg
+        x_btc = torch.empty(2, B, T, Cinp, device=dev, dtype=torch.float16)
+        x_wg = torch.empty(2, B, T, Cinp, device=dev, dtype=bf) if need_w else None
         y = torch.empty(B, Cout, T, device=dev)
         side = None
         if bank is None:
@@ -587,27 +435,17 @@ class _Conv1dTCFn(torch.autograd.Function):
             with side:
                 lib.call("dv3_tc_weightnorm_fwd", _p(v), _p(g), _p(inv), _p(scale), _p(wfwd), 2, _p(wbwd), Cout, Cin,
                          k, _stream())
-        if split:
-            lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, Cin, T, k, dilation, int(causal), 0.0,
-                     None, 0, _stream())
+        lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, Cin, T, k, dilation, int(causal), 0.0,
+                 None, 0, _stream())
         if side is not None:
             side.join()
-        emit = _new_planes(emit_p, training, B, T, Cout, dev, need_bwd)
-        fptr, _keep = _fuse_struct(emit=emit)
         lib.call("dv3_tc_conv", _p(x_btc), _p(wfwd), 2, _p(y), B, Cin, Cout, T, k, dilation, int(causal), 0,
-                 _p(bias), int(relu), 0.0, None, 0, 0, None, None, 0.0, fptr, _stream())
-        rec = None
+                 _p(bias), int(relu), 0.0, None, 0, 0, None, None, 0.0, None, _stream())
         if need_bwd:
             ctx.save_for_backward(v, g, x_wg, wbwd, inv, y if relu else None)
             ctx.cfg = (B, Cin, Cout, T, k, dilation, causal, relu)
             ctx.bias_param = bias if bias.is_leaf else None
             ctx.bank = bank
-            ctx.link = link if (fuse_bwd and link is not None and link.C == Cin) else None
-            if want_rec and fuse_bwd:
-                rec = ProducerRec(POST_RELU if relu else POST_IDENT, Cout, False, y if relu else None)
-                rec.bias_param = ctx.bias_param if (v.is_leaf and g.is_leaf) else None
-            ctx.rec = rec
-        box.append((emit, rec))
         return y
 
     @staticmethod
@@ -620,17 +458,9 @@ class _Conv1dTCFn(torch.autograd.Function):
         need_x = ctx.needs_input_grad[0]
         need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
         sink = _sink(v, g, ctx.bias_param) if (ctx.bias_param is not None and v.is_leaf and g.is_leaf) else None
-        rec = ctx.rec
-        if rec is not None and rec.fused:
-            g_btc = rec.planes
-            dbias = rec.dbias
-            if sink and dbias is not None:
-                sink[2].add_(dbias)
-            rec.planes = rec.a = None
-        else:
-            g_btc = torch.empty(2, B, T, Coutp, device=dev, dtype=bf)
-            dbias = sink[2] if sink else torch.zeros(Cout, device=dev)
-            lib.call("dv3_tc_grad_split", _p(dy), _p(y), _p(g_btc), None, _p(dbias), B, Cout, T, int(relu), _stream())
+        g_btc = torch.empty(2, B, T, Coutp, device=dev, dtype=bf)
+        dbias = sink[2] if sink else torch.zeros(Cout, device=dev)
+        lib.call("dv3_tc_grad_split", _p(dy), _p(y), _p(g_btc), None, _p(dbias), B, Cout, T, int(relu), _stream())
         dv = dg = None
         side = _SideStream(dev)
         if need_w:
@@ -649,27 +479,20 @@ class _Conv1dTCFn(torch.autograd.Function):
         dx = None
         if need_x:
             dx = torch.empty(B, Cin, T, device=dev)
-            fptr = _keep = None
-            link = ctx.link
-            if link is not None and not link.fused and (link.a is not None or link.kind == POST_IDENT):
-                pd = _post_dgrad(link, _rec_sink_bias(link), B, T, dev)
-                fptr, _keep = _fuse_struct(rec=link, dbias=pd)
             lib.call("dv3_tc_conv", _p(g_btc), _p(wbwd), 2, _p(dx), B, Cout, Cin, T, k, dilation, int(causal), 1, None,
-                     0, 0.0, None, 0, 0, None, None, 0.0, fptr, _stream())
+                     0, 0.0, None, 0, 0, None, None, 0.0, None, _stream())
         if need_w:
             side.join()
         if sink:
             dv = dg = dbias = None
-        elif dbias is None:
-            dbias = torch.zeros(Cout, device=dev)
-        return (dx, dv, dg, dbias) + (None,) * 10
+        return (dx, dv, dg, dbias) + (None,) * 4
 
 
 class _ConvT2TCFn(torch.autograd.Function):
     """ConvTranspose1d(k=2,s=2) on the tcgen05 path: a 1x1 conv with 2*Cout rows (j,co) + the time interleave."""
 
     @staticmethod
-    def forward(ctx, x, v, g, bias, xh, link):
+    def forward(ctx, x, v, g, bias):
         _chk(x, v, g, bias)
         B, Cin, T = x.shape
         Cout = v.shape[1]
@@ -681,12 +504,9 @@ class _ConvT2TCFn(torch.autograd.Function):
         wbwd = torch.empty(2, Cin, K2p, device=dev, dtype=bf)
         lib.call("dv3_tc_weightnorm_convt_fwd", _p(v), _p(g), _p(inv), _p(scale), _p(wfwd), 2, _p(wbwd), Cin, Cout,
                  _stream())
-        if _usable(xh, Cin, B, T, 0.0) and xh.wg is not None:
-            x_btc, x_wg = xh.t, xh.wg
-        else:
-            x_btc = torch.empty(2, B, T, Cinp, device=dev, dtype=torch.float16)
-            x_wg = torch.empty(2, B, T, Cinp, device=dev, dtype=bf)
-            lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, Cin, T, 1, 1, 0, 0.0, None, 0, _stream())
+        x_btc = torch.empty(2, B, T, Cinp, device=dev, dtype=torch.float16)
+        x_wg = torch.empty(2, B, T, Cinp, device=dev, dtype=bf)
+        lib.call("dv3_tc_split_input", _p(x), _p(x_btc), 2, _p(x_wg), B, Cin, T, 1, 1, 0, 0.0, None, 0, _stream())
         bias2 = bias.repeat(2)
         yp = torch.empty(B, 2 * Cout, T, device=dev)
         lib.call("dv3_tc_conv", _p(x_btc), _p(wfwd), 2, _p(yp), B, Cin, 2 * Cout, T, 1, 1, 0, 0, _p(bias2), 0, 0.0,
@@ -695,7 +515,6 @@ class _ConvT2TCFn(torch.autograd.Function):
         lib.call("dv3_interleave2", _p(yp), _p(y), B, Cout, T, 0, _stream())
         ctx.save_for_backward(v, g, x_wg, wbwd, inv)
         ctx.cfg = (B, Cin, Cout, T)
-        ctx.link = link if (fuse_bwd and link is not None and link.C == Cin) else None
         return y
 
     @staticmethod
@@ -714,13 +533,8 @@ class _ConvT2TCFn(torch.autograd.Function):
         dx = None
         if ctx.needs_input_grad[0]:
             dx = torch.empty(B, Cin, T, device=dev)
-            fptr = _keep = None
-            link = ctx.link
-            if link is not None and not link.fused and (link.a is not None or link.kind == POST_IDENT):
-                pd = _post_dgrad(link, _rec_sink_bias(link), B, T, dev)
-                fptr, _keep = _fuse_struct(rec=link, dbias=pd)
             lib.call("dv3_tc_conv", _p(g_btc), _p(wbwd), 2, _p(dx), B, 2 * Cout, Cin, T, 1, 1, 0, 1, None, 0, 0.0, None,
-                     0, 0, None, None, 0.0, fptr, _stream())
+                     0, 0, None, None, 0.0, None, _stream())
         dv = dg = None
         if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
             M = 2 * Cout
@@ -731,7 +545,7 @@ class _ConvT2TCFn(torch.autograd.Function):
             lib.call("dv3_tc_wgrad_mn", _p(g_btc), _p(x_wg), _p(partials), numel, B, M, Cin, T, 1, 1, 0, Cout, 2, 1,
                      2 * Cout, 0, _stream())
             dv, dg = _wn_bwd(partials, nsplit, v, g, inv)
-        return dx, dv, dg, dbias, None, None
+        return dx, dv, dg, dbias
 
 
 # 16 keeps the 16-wide speaker projections of the multi-speaker model on tensor cores (measured: vctk step 11.8 -> 10.6 ms)
@@ -755,43 +569,13 @@ def tc_supported(B, C, T, k):
     return bool(lib.raw("dv3_tc_supported")(B, C, T, k))
 
 
-class Chain:
-    """How a conv sits in a sequential stack (modules.run_conv_stack), i.e. what its epilogues may fuse:
-    follows = its input tensor was produced by the previous layer and has no other consumer (-> use the planes /
-    producer record attached to it); emit_p = input dropout of the single consumer of its output (None: the output
-    leaves the stack); want_rec = that consumer may run this op's backward in its data-gradient epilogue."""
-
-    def __init__(self, follows=False, emit_p=None, want_rec=False):
-        self.follows, self.emit_p, self.want_rec = follows, emit_p, want_rec
-
-
-_NO_CHAIN = Chain()
-
-
-def _chain_in(x, chain):
-    if not chain.follows:
-        return None, None
-    return getattr(x, "_dv3_planes", None), getattr(x, "_dv3_rec", None)
-
-
-def _chain_out(y, box):
-    if box:
-        y._dv3_planes, y._dv3_rec = box[0]
-    return y
-
-
 def convblock(x, v, g, bias, spk=None, k=3, dilation=1, causal=False, mode=MODE_GLU, residual=True,
-              p_drop=0.0, training=False, chain=None):
+              p_drop=0.0, training=False):
     """Fused weight-normed dilated conv + gate.  x (B,C,T); v (2C,C,k); g (2C,1,1); bias (2C);
     spk (B,C,T) already softsign'ed (or None)."""
-    chain = chain or _NO_CHAIN
     if conv_math in ("tc", "bf16x3") and x.is_cuda and tc_supported(x.shape[0], x.shape[1], x.shape[2], int(k)):
-        xh, link = _chain_in(x, chain)
-        box = []
-        y = _ConvBlockTCFn.apply(_c(x), v, g, bias, None if spk is None else _c(spk), int(k), int(dilation),
-                                 bool(causal), int(mode), bool(residual), float(p_drop), bool(training), xh,
-                                 chain.emit_p, link, chain.want_rec, box)
-        return _chain_out(y, box)
+        return _ConvBlockTCFn.apply(_c(x), v, g, bias, None if spk is None else _c(spk), int(k), int(dilation),
+                                    bool(causal), int(mode), bool(residual), float(p_drop), bool(training))
     if conv_math not in ("fp32", "bf16x3", "tc"):
         raise Dv3Error("unknown conv_math %r" % (conv_math,))
     return _ConvBlockFn.apply(_c(x), v, g, bias, None if spk is None else _c(spk), int(k), int(dilation),
@@ -839,15 +623,10 @@ class _Conv1dFn(torch.autograd.Function):
         return dx, dv, dg, dbias, None, None, None, None
 
 
-def conv1d(x, v, g, bias, k=1, dilation=1, causal=False, relu=False, chain=None, training=False):
+def conv1d(x, v, g, bias, k=1, dilation=1, causal=False, relu=False):
     """Weight-normed Conv1d with 'same' (or causal) padding, optional fused ReLU.  x (B,Cin,T)."""
     if _use_tc_conv(x, v.shape[1], v.shape[0], k):
-        chain = chain or _NO_CHAIN
-        xh, link = _chain_in(x, chain)
-        box = []
-        y = _Conv1dTCFn.apply(_c(x), v, g, bias, int(k), int(dilation), bool(causal), bool(relu), xh, chain.emit_p,
-                              bool(training), link, chain.want_rec, box)
-        return _chain_out(y, box)
+        return _Conv1dTCFn.apply(_c(x), v, g, bias, int(k), int(dilation), bool(causal), bool(relu))
     return _Conv1dFn.apply(_c(x), v, g, bias, int(k), int(dilation), bool(causal), bool(relu))
 
 
@@ -1041,10 +820,9 @@ class _ConvT2Fn(torch.autograd.Function):
         return dx, dv, dg, dbias
 
 
-def conv_transpose1d_k2s2(x, v, g, bias, chain=None):
+def conv_transpose1d_k2s2(x, v, g, bias):
     if _use_tc_conv(x, v.shape[0], 2 * v.shape[1], 1):
-        xh, link = _chain_in(x, chain or _NO_CHAIN)
-        return _ConvT2TCFn.apply(_c(x), v, g, bias, xh, link)
+        return _ConvT2TCFn.apply(_c(x), v, g, bias)
     return _ConvT2Fn.apply(_c(x), v, g, bias)
 
 

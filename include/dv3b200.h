@@ -223,33 +223,18 @@ int dv3_tc_weightnorm_fwd_batched(const Dv3WnEntry* table_dev, int n, int norm_b
                                   void* stream);
 /* split-K reduction + dg / dv of every record: 1 launch; accumulate = 1 adds into dv / dg. */
 int dv3_weightnorm_bwd_batched(const Dv3WnEntry* table_dev, int n, int bwd_blocks, int accumulate, void* stream);
-/* Work the GEMM epilogues can fuse for the neighbouring ops (NULL = none):
- *  - forward (dv3_tc_convblock_fwd, dv3_tc_conv): np != NULL -> also write the operand planes [2][B][T][np_pitch] of
- *    out * dropmask(np_p, np_seed, np_salt), i.e. what dv3_tc_split_input would produce for the CONSUMER conv
- *    (np_pitch = pad8(channels of this call's output)): np = the fp16 pair its forward GEMM reads, np_wg = the bf16
- *    pair its weight gradient reads (NULL when the consumer needs no weight gradient);
- *  - data gradient (dv3_tc_conv with transpose_taps = 1): post_kind != 0 -> the tensor this call writes is
- *    dL/d(output of a producer op); apply that producer's backward and emit ITS gradient planes + bias-gradient sums:
- *      1 GLU gate, 2 highway gate: post_a / post_s = the producer's saved a, s (post_x = its input, highway only),
- *        post_residual = its residual flag; planes [2][B][T][2*Nc] = [da | db], post_dbias[2*Nc] += sums;
- *      3 ReLU (post_a = the producer's output), 4 identity: planes [2][B][T][pad8(Nc)], post_dbias[Nc] += sums
- *    (what dv3_tc_gate_bwd_split / dv3_tc_grad_split would produce from this call's output). */
-typedef struct Dv3TcFuse {
-    void* np; void* np_wg; const unsigned long long* np_seed; float np_p; unsigned np_salt; int np_pitch;
-    int post_kind, post_residual;
-    const float* post_a; const float* post_s; const float* post_x;
-    void* post_planes; float* post_dbias;
-} Dv3TcFuse;
-/* gated forward: xd = btc planes of dv3_tc_split_input, w = wfwd planes [npl][k][2C][C]. */
+/* gated forward: xd = btc planes of dv3_tc_split_input, w = wfwd planes [npl][k][2C][C].
+ * reserved must be NULL (any other value is refused); it keeps the argument list of ABI version 1. */
 int dv3_tc_convblock_fwd(const void* xd, const void* w, int npl, const float* bias, const float* spk,
                          const float* res, float* y, float* save_a, float* save_s, int B, int C, int T, int k,
-                         int dilation, int causal, int mode, int residual, const Dv3TcFuse* fuse, void* stream);
+                         int dilation, int causal, int mode, int residual, const void* reserved, void* stream);
 /* generic conv / data gradient: out (B,Nc,T) = sum_j A[b,t+off_j,:].W[j,n,:], then *dropmask, +bias, +addend, relu.
- * a: [npl][B][T][pad8(Kc)], w: [npl][k][Nc][pad8(Kc)]; transpose_taps = 1 for a data gradient. */
+ * a: [npl][B][T][pad8(Kc)], w: [npl][k][Nc][pad8(Kc)]; transpose_taps = 1 for a data gradient.
+ * reserved must be NULL, as for dv3_tc_convblock_fwd. */
 int dv3_tc_conv(const void* a, const void* w, int npl, float* out, int B, int Kc, int Nc, int T, int k, int dilation,
                 int causal, int transpose_taps, const float* bias, int relu, float p_drop,
                 const unsigned long long* seed_ptr, unsigned salt, int addmode, const float* e1, const float* e2,
-                float alpha, const Dv3TcFuse* fuse, void* stream);
+                float alpha, const void* reserved, void* stream);
 /* weight gradient from the (B,T,C) planes (MN-major operands, tap shift = TMA row coordinate):
  * dy: [2][B][T][pad8(Mw)], xd: [2][B][T][pad8(Nw)]; partial element (m,n,j) of split s at
  * dw_partials + s*split_stride + (m%msplit)*s_m + (m/msplit)*s_mh + n*s_n + j*s_j; dv3_tc_wgrad_nsplit(...) splits. */

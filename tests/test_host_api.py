@@ -107,17 +107,16 @@ def test_product_never_imports_oracle():
                 assert "import oracle" not in src and "from oracle" not in src, f
 
 
-def test_ctypes_structs_match_the_c_header(tmp_path):
-    """The structs that cross the C ABI by pointer (Dv3WnEntry, Dv3TcFuse, Dv3IncStep, Dv3IncAttn) are mirrored by hand in
+def test_abi_structs_match_the_c_header(tmp_path):
+    """The structs that cross the C ABI by pointer (Dv3WnEntry, Dv3IncStep, Dv3IncAttn) are mirrored by hand in
     ctypes; compile the header with gcc and compare sizeof / every field offset."""
     import ctypes
     import os
     import subprocess
     from deepvoice3_pytorch_b200.weight_bank import Dv3WnEntry
     from deepvoice3_pytorch_b200.incremental import Dv3IncStep, Dv3IncAttn
-    from deepvoice3_pytorch_b200.ops import Dv3TcFuse
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    structs = {"Dv3WnEntry": Dv3WnEntry, "Dv3IncStep": Dv3IncStep, "Dv3IncAttn": Dv3IncAttn, "Dv3TcFuse": Dv3TcFuse}
+    structs = {"Dv3WnEntry": Dv3WnEntry, "Dv3IncStep": Dv3IncStep, "Dv3IncAttn": Dv3IncAttn}
     lines = ['#include <stdio.h>', '#include <stddef.h>', '#include "dv3b200.h"', 'int main(void) {']
     for name, st in structs.items():
         lines.append('printf("%s sizeof %%zu\\n", sizeof(%s));' % (name, name))
@@ -134,6 +133,20 @@ def test_ctypes_structs_match_the_c_header(tmp_path):
         st = structs[name]
         got = ctypes.sizeof(st) if field == "sizeof" else getattr(st, field).offset
         assert got == int(value), "%s.%s: ctypes %d vs C %s" % (name, field, got, value)
+
+
+def test_tc_gemm_entry_points_refuse_a_non_null_reserved_argument():
+    """dv3_tc_convblock_fwd and dv3_tc_conv keep a `reserved` pointer slot in front of `stream`, which must be NULL.
+    Any other value is refused before any device work, so a caller that passes a stream or a pointer there gets an
+    error rather than a launch on the wrong stream."""
+    from deepvoice3_pytorch_b200._lib import lib
+    bad = ctypes.c_void_p(16)
+    rc = lib.raw("dv3_tc_convblock_fwd")(None, None, 2, None, None, None, None, None, None, 1, 128, 128, 3, 1, 0, 0, 1,
+                                         bad, None)
+    assert rc != 0 and "must be NULL" in lib.raw("dv3_last_error")().decode()
+    rc = lib.raw("dv3_tc_conv")(None, None, 2, None, 1, 128, 128, 128, 1, 1, 0, 0, None, 0, 0.0, None, 0, 0, None, None,
+                                0.0, bad, None)
+    assert rc != 0 and "must be NULL" in lib.raw("dv3_last_error")().decode()
 
 
 def test_incremental_stop_rule_matches_reference_loop():
